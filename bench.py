@@ -18,6 +18,10 @@ proposal -> ROI pool -> fc_new_1 -> relation#1 -> fc_new_2 -> relation#2 -> cls/
              training step with 2 images per GPU accumulated before the one allreduce)
   cpu_baseline  the numpy/C oracle of the hot path (oracle/pipeline_np.py) on this host, one image
   --impl reference   the CPU arm: torch-CPU fp32 trunk + oracle hot path, same metric/config (rank 0 only)
+  --dump-outputs DIR what the last timed step returned (either arm), as DIR/<name>.npy
+
+bench.py measures the library as __graft_entry__.build() left it and writes nothing in the tree, which may be read-only: it
+compiles nothing, and stops with an error when the library is missing or older than its sources (run build() first).
 
 Multi-GPU (torchrun): images are independent at test time -> N replicas, one image per rank per step, no data-path
 collective (the reference's only exchange is the gradient allreduce of training; DESIGN.md section "multi-GPU").
@@ -53,7 +57,32 @@ def parse():
     ap.add_argument('--extras-budget', type=float, default=float(os.environ.get('RELNET_EXTRAS_BUDGET_S', '120')),
                     help='seconds the optional blocks (configs[2]/[3], training steps) may take after the headline measurement; past '
                          'it every rank stops and rank 0 prints the line without them')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step returned to its caller as DIR/<name>.npy '
+                         '(float32, float64 for integer outputs; rank 0).  Inputs and weights are seeded, so two builds '
+                         'run with the same arguments can be compared output for output')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(outdir, outputs):
+    """outputs: {name: torch tensor or numpy array} -> outdir/<name>.npy; floating point as float32 (float64 kept), integers
+    as float64 (exact).  The detection outputs of one image are a few MB, far below DUMP_LIMIT."""
+    arrs = {}
+    for k, v in outputs.items():
+        t = torch.as_tensor(v).detach().cpu()
+        arrs[k] = (t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()).numpy()
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError('--dump-outputs: %d bytes exceed the %d byte limit' % (total, DUMP_LIMIT))
+    os.makedirs(outdir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(outdir, k + '.npy'), a)
 
 
 def peaks():
@@ -504,7 +533,7 @@ def run_reference(args):
     trunk = make_trunk('cpu', torch.float32)
     prm = {k: v.numpy() for k, v in init_head_params(0, 'cpu').items()}
     image, im_info = make_inputs()
-    steps = max(1, min(args.steps, 6)); warm = min(args.warmup, 1)       # bounded sample: ~5 s per image on 8 cores
+    steps = args.steps; warm = min(args.warmup, 1)       # ~5 s per image on 8 cores
 
     def step():
         prob, bbox, feat = trunk(image)
@@ -513,10 +542,12 @@ def run_reference(args):
         step()
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        out = step()
     dt = (time.perf_counter() - t0) / steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     v = round(1.0 / dt, 4)
-    sample = 'full step (torch-CPU fp32 trunk + numpy/C oracle hot path), %d timed image(s) of the %d requested' % (steps, args.steps)
+    sample = 'full step (torch-CPU fp32 trunk + numpy/C oracle hot path), %d timed image(s)' % steps
     emit({
         'impl': 'reference', 'metric': 'images/sec', 'value': v, 'unit': 'images/sec', 'n_gpus': args.gpus, 'steps': steps,
         'warmup': warm, 'ms_per_step': round(dt * 1e3, 2), 'higher_is_better': True, 'scaling': 'weak',
@@ -524,6 +555,13 @@ def run_reference(args):
         'config': {'workload': WORKLOAD, 'global_batch': 1, 'parallelism': 'cpu'},
         'cpu_baseline': {'value': v, 'unit': 'images/sec', 'cores': ncores, 'kind': 'port', 'sample': sample},
         'e2e': {'value': v, 'unit': 'images/sec', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}})
+
+
+def require_built():
+    """The tree is measured as build() left it, and may be read-only: nothing is compiled here."""
+    from relnet_b200 import build
+    if not build.current():
+        raise RuntimeError('%s is missing or older than its sources: run __graft_entry__.build() first' % build.LIB)
 
 
 _REAL_STDOUT = None
@@ -546,7 +584,6 @@ def main():
     args = parse()
     if args.impl == 'reference':
         return run_reference(args)
-    import __graft_entry__ as entry
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
     local = int(os.environ.get('LOCAL_RANK', '0'))
@@ -557,11 +594,7 @@ def main():
     if dist_on:
         import torch.distributed as dist
         dist.init_process_group('nccl', device_id=device)
-    if rank == 0:
-        entry.build()
-    if dist_on:
-        import torch.distributed as dist
-        dist.barrier()
+    require_built()
     import relnet_b200
     from relnet_b200 import ops
     from relnet_b200.pipeline import RelationHead, init_head_params
@@ -632,6 +665,8 @@ def main():
     ms = timed(step_resident, args.steps, args.warmup, dist_on)
     if sampler:
         sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, graphed.out)     # the graph's output buffers: what its last replay returned
     ms_e2e_sync = timed(step_e2e, args.steps, max(3, args.warmup // 2), dist_on)
     ms_e2e = timed(step_e2e_stream, args.steps, max(3, args.warmup // 2), dist_on, after=drain)
     ms_hot = timed(step_hot, args.steps, 3, dist_on)

@@ -49,12 +49,18 @@ def _compile(src):
     return src, obj, p.returncode, p.stdout + p.stderr
 
 
+def current():
+    """True when the library exists and was built from the present sources.  Reads only: usable on a read-only tree."""
+    stamp_file = os.path.join(OBJ, 'stamp')
+    return os.path.exists(LIB) and os.path.exists(stamp_file) and open(stamp_file).read() == _stamp()
+
+
 def build(force=False, verbose=False):
+    if not force and current():
+        return LIB
     os.makedirs(OBJ, exist_ok=True)
     stamp_file = os.path.join(OBJ, 'stamp')
     stamp = _stamp()
-    if not force and os.path.exists(LIB) and os.path.exists(stamp_file) and open(stamp_file).read() == stamp:
-        return LIB
     objs, logs = [], []
     with cf.ThreadPoolExecutor(max_workers=min(8, os.cpu_count() or 4)) as ex:
         for src, obj, rc, log in ex.map(_compile, sources()):

@@ -40,8 +40,7 @@ class ClockSampler:
     def start(self): pass
     def summary(self): return {'sm_mhz': 1965}
 bench.ClockSampler = ClockSampler
-import __graft_entry__ as entry
-entry.build = lambda: None
+bench.require_built = lambda: None
 import relnet_b200
 from relnet_b200 import ops, pipeline, trunk as TR, train as TN
 ops.default_precision = lambda: 'f16'

@@ -32,6 +32,77 @@ def test_one_json_line_with_the_contract_keys():
     assert d['train'] == {'graph': True} and d['configs']['3_fpn'] == {'test': 1, 'train': 2} and 'extras' not in d
 
 
+def test_gpu_arm_dump_outputs(tmp_path):
+    """main() hands the graphed step's outputs to --dump-outputs: one float32 .npy per output; the line reports --steps."""
+    import numpy as np
+    d = run(extra=['--steps', '7', '--dump-outputs', str(tmp_path)])
+    assert d['steps'] == 7
+    assert sorted(os.listdir(str(tmp_path))) == ['learn_nms_sorted_bbox.npy', 'nms_final_score_output.npy']
+    a = np.load(str(tmp_path / 'learn_nms_sorted_bbox.npy'))
+    assert a.dtype == np.float32 and a.shape == (100, 80, 4)
+
+
+def test_timed_runs_exactly_steps_between_its_events(monkeypatch):
+    """bench.timed: `warmup` calls before the opening event, exactly `steps` calls between the two events."""
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    state = {'events': 0, 'calls': [0, 0, 0]}                  # calls before / inside / after the timed window
+
+    class Event:
+        def __init__(self, **kw):
+            pass
+
+        def record(self):
+            state['events'] += 1
+
+        def elapsed_time(self, other):
+            return 12.5
+    monkeypatch.setattr(torch.cuda, 'Event', Event)
+    monkeypatch.setattr(torch.cuda, 'synchronize', lambda *a, **k: None)
+
+    def step():
+        state['calls'][state['events']] += 1
+    assert bench.timed(step, 9, 4, False) == 12.5
+    assert state['calls'] == [4, 9, 0]
+
+
+def test_reference_arm_times_every_requested_step(monkeypatch, tmp_path):
+    """--impl reference: the CPU arm times all --steps steps (no cap), reports them, and dumps the last step's outputs."""
+    import argparse
+    import types
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    import relnet_b200  # noqa: F401
+    from relnet_b200 import pipeline, trunk
+    from oracle import pipeline_np
+    calls, marks, lines = [0], [], []
+
+    def head_forward(*a, **k):
+        calls[0] += 1
+        return dict(rois=np.arange(10, dtype=np.int64), cls_score=np.full((3, 4), calls[0], np.float64),
+                    fc_all_2_relu=np.ones((3, 4), np.float16))
+
+    def perf_counter():
+        marks.append(calls[0])
+        return float(len(marks))
+    monkeypatch.setattr(trunk, 'make_trunk', lambda *a, **k: (lambda im: (torch.zeros(1), torch.zeros(1), torch.zeros(1))))
+    monkeypatch.setattr(pipeline, 'init_head_params', lambda *a, **k: {})
+    monkeypatch.setattr(pipeline_np, 'head_forward', head_forward)
+    monkeypatch.setattr(bench, 'cpu_threads', lambda: 1)
+    monkeypatch.setattr(bench, 'time', types.SimpleNamespace(perf_counter=perf_counter))
+    monkeypatch.setattr(bench, 'emit', lines.append)
+    monkeypatch.delenv('RANK', raising=False)
+    bench.run_reference(argparse.Namespace(steps=8, warmup=5, gpus=1, dump_outputs=str(tmp_path)))
+    assert marks == [1, 9] and lines[0]['steps'] == 8                  # one warm-up step, then 8 inside the clock
+    out = {f[:-4]: np.load(str(tmp_path / f)) for f in os.listdir(str(tmp_path))}
+    assert sorted(out) == ['cls_score', 'fc_all_2_relu', 'rois']
+    assert out['rois'].dtype == np.float64 and out['fc_all_2_relu'].dtype == np.float32
+    assert out['cls_score'].dtype == np.float64 and (out['cls_score'] == 9).all()      # the last timed step's outputs
+
+
 def test_failing_optional_block_is_reported_not_fatal():
     d = run({'MOCK_FAIL': '1'})
     assert d['train'] == {'failed': 'boom'} and d['configs']['2_deformable_faster'] == {'images_per_sec': 700}

@@ -3,7 +3,7 @@ read like the calls in the reference's get_symbol bodies and CustomOps."""
 import numpy as np
 import pytest
 import torch
-from conftest import golden, rel_err
+from conftest import golden, golden_rel_err, rel_err
 from oracle import relation_np as R, learn_nms_np as L, proposal_np as P
 
 pytestmark = pytest.mark.gpu
@@ -39,11 +39,12 @@ def test_symbol_methods_bind_like_get_symbol(compat):
     attention_1 = sym.attention_module_multi_head(fc_new_1, position_embedding, nongt_dim=nongt_dim, fc_dim=16,
                                                   feat_dim=1024, index=1, group=16, dim=(1024, 1024, 1024))
     fc_all_1_relu = torch.relu(fc_new_1 + attention_1)
-    assert rel_err(attention_1.cpu().numpy(), g['attention']) < 1e-3
-    assert rel_err(fc_all_1_relu.cpu().numpy(), g['out']) < 1e-3
+    assert golden_rel_err(attention_1.cpu().numpy(), g, 'attention') < 1e-3
+    assert golden_rel_err(fc_all_1_relu.cpu().numpy(), g, 'out') < 1e-3
     # the lazy handles materialise to the reference tensors
-    np.testing.assert_allclose(position_matrix.materialize().cpu().numpy()[:8], g['position_matrix'], rtol=1e-5, atol=1e-5)
-    np.testing.assert_allclose(position_embedding.materialize().cpu().numpy()[:8], g['position_embedding'], atol=2e-4)
+    pm, pe = g['position_matrix'], g['position_embedding']
+    np.testing.assert_allclose(position_matrix.materialize().cpu().numpy()[:len(pm)], pm, rtol=1e-5, atol=1e-5)
+    np.testing.assert_allclose(position_embedding.materialize().cpu().numpy()[:len(pe)], pe, atol=2e-4)
     with pytest.raises(AssertionError):
         sym.attention_module_multi_head(fc_new_1, position_embedding, nongt_dim=nongt_dim, fc_dim=8, group=16)
 
